@@ -3,6 +3,7 @@ bench.py -- env-steps/sec of the batched random-action LocoEnv.step() rollout (B
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--envs 4096] [--task UnitreeA1.simple]
   python bench.py --impl reference ...      # the CPU restatement of the reference loop on the host cores
+  python bench.py --dump-outputs DIR ...    # also write the last timed step's outputs of every workload as DIR/*.npy
 
 Headline workload (BASELINE.json configs[1]): UnitreeA1.simple, 4096 envs per GPU, actions ~ U(-1,1)^12, auto-reset
 from the mini-dataset table; a "step" is one LocoEnv.step() of the whole batch (= 10 MuJoCo sub-steps per env).
@@ -41,6 +42,9 @@ def algo_bytes(eng):
 NCU = json.load(open(os.path.join(ROOT, "profiles", "ncu_constants.json"))) \
     if os.path.exists(os.path.join(ROOT, "profiles", "ncu_constants.json")) else {}
 PREROLL = 40          # untimed steps after the mass reset, so that the timed window sees the stationary episode-age mix
+# array bytes --dump-outputs writes at most (the whole dump, .npy headers included, stays under 64 MB); past it every member
+# keeps the same seeded fraction of its envs
+DUMP_BYTES = 60 * 1024 * 1024
 
 
 def parse():
@@ -58,7 +62,29 @@ def parse():
     p.add_argument("--no-gather", action="store_true", help="N>1: skip the rollout all-gather (it is on by default)")
     p.add_argument("--gather-chunk", type=int, default=0, help="steps per gathered rollout chunk (default: 32, or K/2)")
     p.add_argument("--dr-pool", default=None, help="npz with a domain-randomisation parameter pool (key `pool`)")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write obs / reward / done / next_obs of the last timed step of every workload member (rank 0) "
+                        "as DIR/<workload>.<task>.<array>.npy, float32")
     return p.parse_args()
+
+
+def dump_outputs(out_dir, outputs):
+    """outputs: {prefix: (obs, reward, done, next_obs) numpy arrays of one member}. Writes float32 .npy files; when they
+    would exceed DUMP_BYTES in all, every member keeps a fixed, seeded sample of its envs, listed in <prefix>.env_index.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(x.size * 4 for arrays in outputs.values() for x in arrays)
+    # a sample also writes its env indices (8 bytes per kept env), so the fraction is taken of the total including them
+    frac = 1.0 if total <= DUMP_BYTES else DUMP_BYTES / (total + sum(8 * len(a[0]) for a in outputs.values()))
+    for prefix, arrays in outputs.items():
+        arrays = [np.asarray(x, dtype=np.float32) for x in arrays]
+        n = len(arrays[0])
+        if frac < 1.0:
+            idx = np.sort(np.random.RandomState(0).choice(n, max(1, int(n * frac)), replace=False))
+            arrays = [x[idx] for x in arrays]
+            np.save(os.path.join(out_dir, prefix + ".env_index.npy"), idx.astype(np.float64))
+        for name, x in zip(("obs", "reward", "done", "next_obs"), arrays):
+            np.save(os.path.join(out_dir, "%s.%s.npy" % (prefix, name)), x)
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -213,6 +239,10 @@ class Workload:
     def launches(self):
         return sum(e.launches for e in self.engines)
 
+    def named_outputs(self, tag):
+        """{"<tag>.<task>": (obs, reward, done, next_obs)} of the last step that `measure` timed."""
+        return {"%s.%s" % (tag, t): o for (t, _, _), o in zip(self.members, self.last_outputs)}
+
     def step(self, acts, packed=None):
         if len(self.engines) == 1:
             return [self.engines[0].step(acts[0], auto_reset=True, packed=None if packed is None else packed[0])]
@@ -239,10 +269,11 @@ class Workload:
             torch.cuda.synchronize()
 
         def one_step(k):
-            self.step([x[k] for x in actions], None if rg is None else [g.slot() for g in rg])
+            out = self.step([x[k] for x in actions], None if rg is None else [g.slot() for g in rg])
             if rg is not None:
                 for g in rg:
                     g.advance()
+            return out
 
         for k in range(PREROLL + W):
             one_step(k)
@@ -266,7 +297,7 @@ class Workload:
                 flush.fill_(k & 0xff)
             f1[k].record()
             s0[k].record()
-            one_step(PREROLL + W + k)
+            last = one_step(PREROLL + W + k)
             s1[k].record()
         if rg is not None:
             for g in rg:
@@ -274,6 +305,8 @@ class Workload:
         t_end.record()
         barrier()
         clocks = sampler.stop() if sampler else None
+        if a.dump_outputs:                      # per member (obs, reward, done, next_obs) of the last timed step
+            self.last_outputs = [tuple(x.cpu().numpy() for x in r) for r in last]
         span = t_start.elapsed_time(t_end)
         flush_ms = sum(x.elapsed_time(y) for x, y in zip(f0, f1))
         kernel_ms = sum(x.elapsed_time(y) for x, y in zip(s0, s1))
@@ -302,7 +335,8 @@ class Workload:
         from loco_mujoco_b200.parallel import aggregate_throughput
         dev, K = self.dev, a.steps
         envs = self.batch.envs
-        h_act = [(torch.rand((K, e.n_envs, e.action_dim)) * 2 - 1).pin_memory() for e in self.engines]
+        gen = torch.Generator().manual_seed(4321 + int(os.environ.get("RANK", "0")))
+        h_act = [(torch.rand((K, e.n_envs, e.action_dim), generator=gen) * 2 - 1).pin_memory() for e in self.engines]
         d_act = [torch.empty((e.n_envs, e.action_dim), dtype=torch.float32, device=dev) for e in self.engines]
         h_out = [torch.empty_like(e.packed_out, device="cpu").pin_memory() for e in self.engines]
         h_nxt = [torch.empty_like(e.next_obs, device="cpu").pin_memory() for e in self.engines]
@@ -416,6 +450,7 @@ def main():
     head = Workload(a.task, [(a.task, a.envs, {})], rank, world, local, pools)
     gather = world > 1 and not a.no_gather
     res = head.measure(a, rank, gather, sampler_index=local)
+    dumps = head.named_outputs("head") if a.dump_outputs else {}
     res_nog = head.measure(a, rank, False) if gather else None
     e2e = head.measure_e2e(a)
     line = None
@@ -450,6 +485,8 @@ def main():
         for name, members in plan:
             wl = Workload(name, members, rank, world, local)
             r = wl.measure(a, rank, gather)
+            if a.dump_outputs:
+                dumps.update(wl.named_outputs(name.split(":")[0].replace(" ", "")))
             e = wl.measure_e2e(a)
             extra = {}
             if members[0][0].startswith("HumanoidTorque") and len(members) == 1:
@@ -484,6 +521,8 @@ def main():
             line["cpu_baseline"] = cpu
         else:
             line["cpu_baseline"] = None
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

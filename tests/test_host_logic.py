@@ -82,22 +82,16 @@ def test_taskspec_pack_layout(bundled_only):
     assert mi[0] == 0x4C4F434F and mi[2] == env._model.nbody and mi[3] == 18
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/loco_mujoco"), reason="needs the reference checkout")
-def test_bundled_assets_match_live_compile():
-    import subprocess, sys
-    code = ("import numpy as np, os;"
-            "from loco_mujoco_b200 import LocoEnv, modelpack;"
-            "e = LocoEnv.make('UnitreeA1.simple.real', debug=True);"
-            "a = modelpack.pack(e._model); t = e.task_spec().pack();"
-            "np.savez('/tmp/_ls_%s.npz' % os.environ.get('TAG'), a0=a[0], a1=a[1], t0=t[0], t1=t[1])")
-    env = dict(os.environ, PYTHONPATH=ROOT, TAG="live")
-    env.pop("LOCO_MUJOCO_B200_FORCE_BUNDLED", None)
-    subprocess.check_call([sys.executable, "-c", code], env=env)
-    env2 = dict(env, TAG="bundled", LOCO_MUJOCO_B200_FORCE_BUNDLED="1")
-    subprocess.check_call([sys.executable, "-c", code], env=env2)
-    a, b = np.load("/tmp/_ls_live.npz"), np.load("/tmp/_ls_bundled.npz")
-    for k in a.files:
-        assert np.array_equal(a[k], b[k]), k
+def test_bundled_assets_match_live_compile(bundled_only):
+    """The bundled UnitreeA1.simple asset packs to exactly the ModelPack / TaskSpec blobs that a live compile of a
+    loco-mujoco checkout gives (MJCF + mini dataset; LOCO_MUJOCO_PATH set, bundled assets not forced), stored in
+    tests/golden/UnitreeA1.simple.live_compile.npz as a0, a1 (modelpack.pack) and t0, t1 (TaskSpec.pack)."""
+    from loco_mujoco_b200 import modelpack
+    e = make_env("UnitreeA1.simple")
+    a, t = modelpack.pack(e._model), e.task_spec().pack()
+    live = np.load(os.path.join(ROOT, "tests", "golden", "UnitreeA1.simple.live_compile.npz"))
+    for k, x in zip(("a0", "a1", "t0", "t1"), (*a, *t)):
+        assert np.array_equal(live[k], x), k
 
 
 def test_taskspec_layout_and_feature_sources(bundled_only):
